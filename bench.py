@@ -56,15 +56,16 @@ def dram_ceiling_tok_s(bytes_per_token: float) -> dict:
 
 
 def model_dir() -> Path:
+    name = f"minigpt4_b200_models-{os.getuid()}"   # per account: a directory another user created is not writable here
     for cand in ("/dev/shm", "/tmp"):
         try:
             if shutil.disk_usage(cand).free > 12 << 30:
-                d = Path(cand) / "minigpt4_b200_models"
+                d = Path(cand) / name
                 d.mkdir(parents=True, exist_ok=True)
                 return d
         except OSError:
             pass
-    d = Path("/tmp/minigpt4_b200_models")
+    d = Path("/tmp") / name
     d.mkdir(parents=True, exist_ok=True)
     return d
 
@@ -264,10 +265,17 @@ def main():
     ap.add_argument("--cpu-tokens", type=int, default=0, help="decode tokens of the CPU legs (default: 32)")
     ap.add_argument("--cpu-encode-every-step", action="store_true")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (image embedding, chat reply, "
+                                                          "greedy ids, last logits) as DIR/<name>.npy, float32 / float64; the inputs are seeded, "
+                                                          "so two builds can be compared output for output")
     ap.add_argument("--mode", default="replicas", choices=["replicas", "tp"],
                     help="N>1: 'replicas' = one independent decode stream per GPU, no data-path collective (weak scaling, default); "
                          "'tp' = one stream, LLaMA layers tensor-parallel over the GPUs with an NCCL sum per row-split matmul (strong scaling)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: --impl ours only")
     global N_GEN
     N_GEN = args.tokens
     if args.impl == "reference":
@@ -315,8 +323,8 @@ def main():
             import torch
             torch.cuda.synchronize(); dist.barrier(); torch.cuda.synchronize()
 
-    def step(timed: bool):
-        """returns dict: encode_dev_ms, chain_ms, turn_s (whole turn through the ABI), ttft_s, decode_s, ids"""
+    def step(timed: bool, keep_embedding: bool = False):
+        """returns dict: encode_dev_ms, chain_ms, turn_s (whole turn through the ABI), ttft_s, decode_s, ids (+ a copy of the image embedding)"""
         # -- e2e leg: ONE chat turn through the reference ABI with host buffers, wall clock around all of it:
         #    image H2D + encode + embedding D2H | system prompt | embedding H2D + prefix + prompt | 128 x (decode step + 4-byte D2H + id_to_token)
         lib.minigpt4_reset_chat(ctx)
@@ -336,9 +344,10 @@ def main():
         rows = np.ctypeslib.as_array(emb.data, shape=(emb.n_embeddings,)).reshape(32, -1)
         tp0 = time.perf_counter(); ext.eval_embd(ctx, rows); ext.flush(ctx); prefix_ms = (time.perf_counter() - tp0) * 1e3
         ids, chain_ms = ext.decode_chain(ctx, N_GEN)
+        kept = rows.copy() if keep_embedding else None
         lib.minigpt4_free_embedding(emb)
         return {"enc_dev": enc_dev, "enc_wall": (t_enc - t0) * 1e3, "chain_ms": chain_ms, "turn_s": t_end - t0, "ttft_s": t_first - t0,
-                "prefill_s": t_pre - t_enc, "decode_s": t_end - t_pre, "prefix_ms": prefix_ms, "ids": ids, "toks": toks}
+                "prefill_s": t_pre - t_enc, "decode_s": t_end - t_pre, "prefix_ms": prefix_ms, "ids": ids, "toks": toks, "emb": kept}
 
     for _ in range(args.warmup):
         step(False)
@@ -347,11 +356,20 @@ def main():
     barrier()
     sampler.start()
     t_begin = time.perf_counter()
-    res = [step(True) for _ in range(args.steps)]
+    res = [step(True, keep_embedding=bool(args.dump_outputs) and i == args.steps - 1) for i in range(args.steps)]
     barrier()
     wall = time.perf_counter() - t_begin
     clocks = sampler.stop()
     launches = ext.stats(ctx).kernel_launches - launches0
+    if args.dump_outputs and rank == 0:
+        # what the last timed step handed its caller, read before anything else runs on the context
+        out = Path(args.dump_outputs)
+        out.mkdir(parents=True, exist_ok=True)
+        last = res[-1]
+        np.save(out / "image_embedding.npy", last["emb"].astype(np.float32))                       # minigpt4_encode_image, [32, n_embd]
+        np.save(out / "chat_reply_codepoints.npy", np.array([ord(c) for c in "".join(last["toks"])], np.float64))  # N_GEN x minigpt4_end_chat_image
+        np.save(out / "decode_ids.npy", last["ids"].astype(np.float64))                            # device-chained greedy ids, [N_GEN]
+        np.save(out / "decode_logits.npy", ext.logits(ctx).astype(np.float32))                     # logits of the last chained step, [n_vocab]
 
     chain_ms = sum(r["chain_ms"] for r in res); turn_s = sum(r["turn_s"] for r in res); dec_s = sum(r["decode_s"] for r in res)
     enc_dev = float(np.mean([r["enc_dev"] for r in res])); enc_wall = float(np.mean([r["enc_wall"] for r in res]))

@@ -75,17 +75,31 @@ def test_quantize_missing_input(lib):
 
 
 def test_reference_binding_binds_unmodified(lib):
-    """The reference's own ctypes file (when mounted) must bind to the new .so without edits."""
-    ref = Path("/root/reference/minigpt4/minigpt4_library.py")
-    if not ref.exists():
-        pytest.skip("reference tree not mounted on this box")
-    import importlib.util
-    from minigpt4_cpp_b200.build import OUT
-    spec = importlib.util.spec_from_file_location("ref_minigpt4_library", ref)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    rlib = mod.MiniGPT4SharedLibrary(str(OUT))
-    assert rlib.minigpt4_is_eos("x###") and rlib.minigpt4_contains_eos_token("##")
+    """The original project's ctypes binding (minigpt4/minigpt4_library.py) must bind to the new .so without edits.  What it
+    declares - every prototype, both struct layouts - and what its GPU-free calls returned are recorded in
+    tests/golden/reference_binding.json (tools/make_reference_fixtures.py); here they are applied to the library as the binding does."""
+    import json
+    import minigpt4_cpp_b200 as m
+    rec = json.loads((ROOT / "tests" / "golden" / "reference_binding.json").read_text())
+    ours = {"MiniGPT4Image": m.MiniGPT4Image, "MiniGPT4Embedding": m.MiniGPT4Embedding}
+    for name, s in rec["structs"].items():
+        S = ours[name]
+        assert ctypes.sizeof(S) == s["size"]
+        assert [[f, t.__name__, getattr(S, f).offset] for f, t in S._fields_] == s["fields"], name
+    types = {t.__name__: t for t in (ctypes.c_int, ctypes.c_float, ctypes.c_void_p, ctypes.c_ulong)}
+    types.update(LP_c_char=ctypes.POINTER(ctypes.c_char), LP_LP_c_char=ctypes.POINTER(ctypes.POINTER(ctypes.c_char)),
+                 LP_c_float=ctypes.POINTER(ctypes.c_float), LP_MiniGPT4Image=ctypes.POINTER(m.MiniGPT4Image),
+                 LP_MiniGPT4Embedding=ctypes.POINTER(m.MiniGPT4Embedding))
+    L = ctypes.cdll.LoadLibrary(lib.library._name)  # its own handle, like the binding's: these prototypes stay out of the session-wide one
+    assert len(rec["prototypes"]) == 18
+    for name, p in rec["prototypes"].items():
+        fn = getattr(L, name)
+        if p["argtypes"] is not None:
+            fn.argtypes = [types[t] for t in p["argtypes"]]
+        fn.restype = None if p["restype"] is None else types[p["restype"]]
+    for name, cases in rec["calls"].items():
+        for s, want in cases.items():
+            assert bool(getattr(L, name)(s.encode("utf-8"))) == want, (name, s)
 
 
 def test_null_arguments_are_harmless(lib):
