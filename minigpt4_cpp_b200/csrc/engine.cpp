@@ -127,7 +127,6 @@ Error Engine::add_tokens(const std::vector<int32_t> &tokens) {
     for (int i = 0; ok && i < n; ++i) if (tokens[(size_t)i] < 0 || tokens[(size_t)i] >= n_vocab) { MG4_ERR("token id %d out of range", tokens[(size_t)i]); ok = false; }
     if (ok) {
         if (n == 1 && pend_ids_.empty()) ok = llm_->decode_step(tokens[0], n_past_);   // asynchronous: the next sample / flush synchronises
-        else if (!llm_->rows_mergeable()) ok = flush() && llm_->eval_tokens(tokens.data(), n, n_past_);
         else {
             for (int i = 0; ok && i < n; i += kMaxPending) {   // a queue never exceeds kMaxPending rows
                 const int c = std::min(kMaxPending, n - i);
@@ -148,17 +147,12 @@ Error Engine::add_embedding(const float *rows, int n_rows) {
     if (n_rows <= 0) return ErrNone;
     const size_t E = (size_t)llm_->dims().n_embd;
     bool ok = n_rows <= kMaxPending && n_past_ + n_rows <= llm_->dims().n_ctx;
+    if (ok && (int)pend_ids_.size() + n_rows > kMaxPending) ok = flush();
     if (ok) {
-        if (!llm_->rows_mergeable()) ok = flush() && llm_->eval_embd(rows, n_rows, n_past_);
-        else {
-            if ((int)pend_ids_.size() + n_rows > kMaxPending) ok = flush();
-            if (ok) {
-                if (pend_ids_.empty()) pend_base_ = n_past_;
-                const int k0 = (int)(pend_emb_.size() / E);
-                for (int i = 0; i < n_rows; ++i) pend_ids_.push_back(-1 - (k0 + i));
-                pend_emb_.insert(pend_emb_.end(), rows, rows + (size_t)n_rows * E);
-            }
-        }
+        if (pend_ids_.empty()) pend_base_ = n_past_;
+        const int k0 = (int)(pend_emb_.size() / E);
+        for (int i = 0; i < n_rows; ++i) pend_ids_.push_back(-1 - (k0 + i));
+        pend_emb_.insert(pend_emb_.end(), rows, rows + (size_t)n_rows * E);
     }
     if (!ok) { MG4_ERR("Failed to add embedding"); return ErrFailedToAddEmbedding; }
     n_past_ += n_rows;

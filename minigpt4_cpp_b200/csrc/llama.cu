@@ -284,6 +284,20 @@ void LlamaDevice::launch_layers(int nt, int ntok, bool want_logits) {
     const bool tp = tp_ && tp_->world > 1;
     const float kq_scale = 1.0f / sqrtf((float)d_.n_embd / (float)d_.n_head);
     const size_t attn_smem = (size_t)C * 6;
+    // wo / down: x_ += W x, the residual added in the matvec epilogue or, under tensor parallelism, after the partial sums are all-reduced
+    auto matvec_resid = [&](const QMat &w, const float *x, int x_stride) {
+        MatvecArgs b{};
+        b.w = w; b.x = x; b.x_stride = x_stride; b.norm_w = nullptr; b.ntok = ntok; b.n_valid = b.w.rows; b.state = state_; b.tab_silu = tab_silu_; b.staged = qact_;
+        if (!tp) { b.epi = EPI_RESID; b.out = x_; b.out_stride = E; b.resid = x_; launch_matvec(b, nt, sm_count_, stream_, &launches_); }
+        else if (tp_->peers_ready()) {   // partial -> this rank's exchange buffer; ONE kernel: signal peers, wait, sum all partials + residual out of peer memory
+            b.epi = EPI_PLAIN; b.out = tp_->partial_out(); b.out_stride = E; launch_matvec(b, nt, sm_count_, stream_, &launches_);
+            tp_->all_reduce_resid(x_, x_, (size_t)ntok * E, stream_); ++launches_;
+        } else {
+            b.epi = EPI_PLAIN; b.out = partial_; b.out_stride = E; launch_matvec(b, nt, sm_count_, stream_, &launches_);
+            tp_->all_reduce_sum(partial_, (size_t)ntok * E, stream_);
+            add_kernel<<<(ntok * E + 255) / 256, 256, 0, stream_>>>(x_, partial_, ntok * E); ++launches_;
+        }
+    };
     for (int il = 0; il < d_.n_layer; ++il) {
         Layer &L = layers_[(size_t)il];
         __half *kc = kcache_ + (size_t)il * C * El, *vc = vcache_ + (size_t)il * C * El;
@@ -300,33 +314,12 @@ void LlamaDevice::launch_layers(int nt, int ntok, bool want_logits) {
         }
         attn_kernel<<<dim3((unsigned)n_head_local_, (unsigned)ntok), 256, attn_smem, stream_>>>(q_, kc, vc, att_, state_, El, C, kq_scale, tab_exp_);
         CUDA_CHECK(cudaGetLastError()); ++launches_;
-
-        MatvecArgs b{};
-        b.w = L.wo; b.x = att_; b.x_stride = El; b.norm_w = nullptr; b.ntok = ntok; b.n_valid = b.w.rows; b.state = state_; b.tab_silu = tab_silu_; b.staged = qact_;
-        if (!tp) { b.epi = EPI_RESID; b.out = x_; b.out_stride = E; b.resid = x_; launch_matvec(b, nt, sm_count_, stream_, &launches_); }
-        else if (tp_->peers_ready()) {   // partial -> this rank's exchange buffer; ONE kernel: signal peers, wait, sum all partials + residual out of peer memory
-            b.epi = EPI_PLAIN; b.out = tp_->partial_out(); b.out_stride = E; launch_matvec(b, nt, sm_count_, stream_, &launches_);
-            tp_->all_reduce_resid(x_, x_, (size_t)ntok * E, stream_); ++launches_;
-        } else {
-            b.epi = EPI_PLAIN; b.out = partial_; b.out_stride = E; launch_matvec(b, nt, sm_count_, stream_, &launches_);
-            tp_->all_reduce_sum(partial_, (size_t)ntok * E, stream_);
-            add_kernel<<<(ntok * E + 255) / 256, 256, 0, stream_>>>(x_, partial_, ntok * E); ++launches_;
-        }
+        matvec_resid(L.wo, att_, El);
         MatvecArgs c{};
         c.w = L.w13; c.x = x_; c.x_stride = E; c.norm_w = L.ffn_norm; c.ntok = ntok; c.epi = EPI_SWIGLU; c.out = act_; c.out_stride = FFl; c.n_valid = c.w.rows;
         c.state = state_; c.tab_silu = tab_silu_; c.staged = qact_;
         launch_matvec(c, nt, sm_count_, stream_, &launches_);
-        MatvecArgs e{};
-        e.w = L.w2; e.x = act_; e.x_stride = FFl; e.norm_w = nullptr; e.ntok = ntok; e.n_valid = e.w.rows; e.state = state_; e.tab_silu = tab_silu_; e.staged = qact_;
-        if (!tp) { e.epi = EPI_RESID; e.out = x_; e.out_stride = E; e.resid = x_; launch_matvec(e, nt, sm_count_, stream_, &launches_); }
-        else if (tp_->peers_ready()) {   // partial -> this rank's exchange buffer; ONE kernel: signal peers, wait, sum all partials + residual out of peer memory
-            e.epi = EPI_PLAIN; e.out = tp_->partial_out(); e.out_stride = E; launch_matvec(e, nt, sm_count_, stream_, &launches_);
-            tp_->all_reduce_resid(x_, x_, (size_t)ntok * E, stream_); ++launches_;
-        } else {
-            e.epi = EPI_PLAIN; e.out = partial_; e.out_stride = E; launch_matvec(e, nt, sm_count_, stream_, &launches_);
-            tp_->all_reduce_sum(partial_, (size_t)ntok * E, stream_);
-            add_kernel<<<(ntok * E + 255) / 256, 256, 0, stream_>>>(x_, partial_, ntok * E); ++launches_;
-        }
+        matvec_resid(L.w2, act_, FFl);
     }
     if (want_logits) {
         MatvecArgs o{};
@@ -340,26 +333,10 @@ void LlamaDevice::launch_layers(int nt, int ntok, bool want_logits) {
     if (want_logits) CUDA_CHECK(cudaMemcpyAsync(h_argmax_, &state_->argmax_id, 4, cudaMemcpyDeviceToHost, stream_));
 }
 
-void LlamaDevice::run_chunk(int n, bool want_logits, bool from_tokens) {
-    // h_state_ already holds n_past / n_tok / tokens for this chunk
-    CUDA_CHECK(cudaMemcpyAsync(state_, h_state_, offsetof(DeviceState, argmax_key), cudaMemcpyHostToDevice, stream_));
-    if (from_tokens) {
-        if (tok_type_ == GG_Q4_K) embed_q4k_kernel<<<n, 256, 0, stream_>>>((const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, state_, x_);
-        else if (tok_type_ == GG_Q5_0 || tok_type_ == GG_Q5_1 || tok_type_ == GG_Q8_0) embed_b32_kernel<<<n, 256, 0, stream_>>>(tok_type_, (const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, state_, x_);
-        else embed_kernel<<<n, 256, 0, stream_>>>(tok_type_, (const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, state_, x_);
-        ++launches_;
-    }
-    launch_layers(nt_for(n), n, want_logits);
-    CUDA_CHECK(cudaStreamSynchronize(stream_));  // h_state_ is rewritten by the next chunk
-}
-
 // One or more passes over `n` mixed rows starting at position n_past: ids[i] >= 0 is a token, ids[i] < 0 is row -1 - ids[i] of emb_host
 // (n_emb rows of n_embd floats).  The engine collects consecutive add_tokens / add_embedding calls of a chat turn (reference call sites
 // minigpt4.cpp:2365-2382 and :2399-2415 evaluate each piece separately; results are batch invariant) and evaluates them together, so the
 // weights stream once per kPrefillMax rows instead of once per piece.
-bool LlamaDevice::rows_mergeable() const {
-    return tok_type_ == GG_F32 || tok_type_ == GG_F16 || tok_type_ == GG_Q4_0 || tok_type_ == GG_Q4_1 || tok_type_ == GG_Q5_K || tok_type_ == GG_Q6_K;
-}
 bool LlamaDevice::eval_rows(const int32_t *ids, int n, const float *emb_host, int n_emb, int n_past) {
     if (n <= 0) return true;
     if (n_past + n > d_.n_ctx) { MG4_ERR("context overflow: %d + %d > n_ctx %d", n_past, n, d_.n_ctx); return false; }
@@ -372,7 +349,6 @@ bool LlamaDevice::eval_rows(const int32_t *ids, int n, const float *emb_host, in
         const bool last = i + c == n;
         CUDA_CHECK(cudaStreamSynchronize(stream_));  // h_state_ (pinned) of the previous pass / decode step has been consumed
         h_state_->n_past = n_past + i; h_state_->n_tok = c;
-        for (int j = 0; j < std::min(c, 8); ++j) h_state_->tokens[j] = ids[i + j] >= 0 ? ids[i + j] : 0;
         CUDA_CHECK(cudaMemcpyAsync(state_, h_state_, offsetof(DeviceState, argmax_key), cudaMemcpyHostToDevice, stream_));
         CUDA_CHECK(cudaMemcpyAsync(tok_ids_, ids + i, (size_t)c * 4, cudaMemcpyHostToDevice, stream_));
         embed_rows_kernel<<<c, 256, 0, stream_>>>(tok_type_, (const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, tok_ids_, embd_in_, x_);
@@ -381,37 +357,6 @@ bool LlamaDevice::eval_rows(const int32_t *ids, int n, const float *emb_host, in
         else launch_layers(nt_for(c), c, last);
     }
     CUDA_CHECK(cudaStreamSynchronize(stream_));
-    return true;
-}
-bool LlamaDevice::eval_tokens(const int32_t *ids, int n, int n_past) {
-    if (n <= 0) return true;
-    if (rows_mergeable()) return eval_rows(ids, n, nullptr, 0, n_past);
-    if (n_past + n > d_.n_ctx) { MG4_ERR("context overflow: %d + %d > n_ctx %d", n_past, n, d_.n_ctx); return false; }
-    for (int i = 0; i < n; ++i) if (ids[i] < 0 || ids[i] >= d_.n_vocab) { MG4_ERR("token id %d out of range", ids[i]); return false; }
-    for (int i = 0; i < n; i += 8) {   // token-embedding types outside dequant_elem (experimental block types): per-op path, 8 rows per pass
-        const int c = std::min(8, n - i);
-        h_state_->n_past = n_past + i; h_state_->n_tok = c;
-        for (int j = 0; j < c; ++j) h_state_->tokens[j] = ids[i + j];
-        run_chunk(c, i + c == n, true);
-    }
-    return true;
-}
-bool LlamaDevice::eval_embd(const float *rows_host, int n, int n_past) {
-    if (n <= 0) return true;
-    if (n > 512) { MG4_ERR("eval_embd: at most 512 rows per call"); return false; }
-    if (n_past + n > d_.n_ctx) { MG4_ERR("context overflow: %d + %d > n_ctx %d", n_past, n, d_.n_ctx); return false; }
-    if (rows_mergeable()) {
-        std::vector<int32_t> ids((size_t)n);
-        for (int i = 0; i < n; ++i) ids[(size_t)i] = -1 - i;
-        return eval_rows(ids.data(), n, rows_host, n, n_past);
-    }
-    CUDA_CHECK(cudaMemcpyAsync(embd_in_, rows_host, (size_t)n * d_.n_embd * 4, cudaMemcpyHostToDevice, stream_));
-    for (int i = 0; i < n; i += 8) {
-        const int c = std::min(8, n - i);
-        h_state_->n_past = n_past + i; h_state_->n_tok = c;
-        CUDA_CHECK(cudaMemcpyAsync(x_, embd_in_ + (size_t)i * d_.n_embd, (size_t)c * d_.n_embd * 4, cudaMemcpyDeviceToDevice, stream_));
-        run_chunk(c, i + c == n, false);
-    }
     return true;
 }
 void LlamaDevice::logits_to_host(float *dst) {
@@ -473,11 +418,9 @@ static void pq_build(PQMat &p, const QMat &m) {
 bool LlamaDevice::build_prefill() {
     if (getenv("MINIGPT4_B200_NO_PREFILL_GEMM")) return false;
     if (tp_ && tp_->world > 1) return false;  // (tensor-parallel ranks keep the per-op prefill path for now)
-    if (!(tok_type_ == GG_F32 || tok_type_ == GG_F16 || tok_type_ == GG_Q4_0 || tok_type_ == GG_Q4_1 || tok_type_ == GG_Q5_K || tok_type_ == GG_Q6_K)) return false;
-    for (auto &L : layers_) {
+    for (auto &L : layers_) {   // (each matrix stages its own input: mixed Q4_0 / Q4_1 layers are fine)
         if (!L.fused_qkv) return false;
         for (const QMat *m : {&L.qkv, &L.wo, &L.w13, &L.w2}) if (m->type != GG_Q4_0 && m->type != GG_Q4_1) return false;
-        if (act_of(L.qkv.type) != act_of(L.w13.type)) {}  // (each matrix stages its own input: mixed Q4_0 / Q4_1 layers are fine)
     }
     const int E = d_.n_embd, FF = d_.n_ff;
     size_t free_b = 0, total_b = 0; CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
@@ -497,7 +440,6 @@ bool LlamaDevice::build_prefill() {
     const size_t smem = 1024 + (size_t)pf::kStages * pf::kStageBytes + pf::kStackBytes + 256;
     CUDA_CHECK(cudaFuncSetAttribute(pf::prefill_gemm_q4<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_CHECK(cudaFuncSetAttribute(pf::prefill_gemm_q4<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CUDA_CHECK(cudaFuncSetAttribute(attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, std::max(49152, d_.n_ctx * 6)));
     CUDA_CHECK(cudaDeviceSynchronize());
     MG4_INFO("tensor-core prefill: int8 class-major operand cache built (%d / %d slots per class)", pf_S_e_, pf_S_ff_);
     return true;
@@ -577,6 +519,8 @@ bool LlamaDevice::build_mega() {
     const int wt = output_.type;
     if (wt != GG_Q4_0 && wt != GG_Q4_1 && wt != GG_Q5_K) return false;   // homogeneous Q4_0 / Q4_1 / Q5_K files (the reference README's q5_k download has a Q6_K output matrix: per-op path)
     for (auto &L : layers_) if (!L.fused_qkv || L.qkv.type != wt || L.wo.type != wt || L.w13.type != wt || L.w2.type != wt) return false;
+    // OP_EMBED gathers through dequant_elem, which has no Q4_K / Q5_0 / Q5_1 / Q8_0 case (such tok_embeddings: per-op graph)
+    if (tok_type_ != GG_F32 && tok_type_ != GG_F16 && tok_type_ != GG_Q4_0 && tok_type_ != GG_Q4_1 && tok_type_ != GG_Q5_K && tok_type_ != GG_Q6_K) return false;
     if (d_.n_embd % 256 || d_.n_ff % 32 || d_.n_embd > 1024 * mk6::kNormItems || d_.n_ff > 4 * mk6::kConsumerThreads * mk6::kPlainItems) return false;
     if (d_.head_dim != 128 || d_.n_head > sm_count_ || 7 * d_.n_layer + 3 > mk6::kMaxOps) return false;
     if (tp && (n_embd_local_ % 32 || n_ff_local_ % 32)) return false;
@@ -587,20 +531,9 @@ bool LlamaDevice::build_mega() {
     CUDA_CHECK(cudaMalloc((void **)&mega_barrier_, 64)); CUDA_CHECK(cudaMemset(mega_barrier_, 0, 64));
     mega_n_ops_ = (tp ? 7 : 5) * d_.n_layer + 3;
     if (getenv("MINIGPT4_B200_MEGA_TRACE")) { CUDA_CHECK(cudaMalloc((void **)&mega_trace_, (size_t)(mega_n_ops_ + 1) * 32 * sizeof(long long))); CUDA_CHECK(cudaMemset(mega_trace_, 0, (size_t)(mega_n_ops_ + 1) * 32 * sizeof(long long))); }
-    mega_gen_ = 6;
-    if (!build_mega6()) return false;
-    const void *fn = mega_fn();
-    CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mega_smem_));
-    int occ = 0;
-    CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, mk6::kThreads, mega_smem_));
-    if (occ < 1) { MG4_ERR("megakernel does not fit on an SM (smem %zu)", mega_smem_); return false; }
-    return true;
-}
 
-// generation 6: self-refilled per-warp streams (llama_mega6.cuh)
-bool LlamaDevice::build_mega6() {
+    // generation 6: self-refilled per-warp streams (llama_mega6.cuh)
     using namespace mk6;
-    const bool tp = tp_ && tp_->world > 1;
     const int E = d_.n_embd, FF = n_ff_local_;   // (tensor parallel: this rank's feed-forward columns)
     size_t act_b = mega_type_ == GG_Q5_K ? std::max(act_bytes(ACT_Q8_K, FF), act_bytes(ACT_Q8_K, E)) : std::max(act6_bytes(FF), act6_bytes(E));
     act_b = std::max(act_b, (size_t)d_.n_ctx * 6);  // the attention op (which stages no activations) uses the region as its scratch
@@ -610,7 +543,7 @@ bool LlamaDevice::build_mega6() {
     // a slot holds a row pair of an n_embd-wide matrix or ONE row of an n_ff-wide matrix (whose pair then takes both slots of the warp)
     int slot = std::max(2 * rb_e, rb_ff);
     slot = (slot + 15) & ~15;
-    cudaDeviceProp prop; int dev = 0; CUDA_CHECK(cudaGetDevice(&dev)); CUDA_CHECK(cudaGetDeviceProperties(&prop, dev));
+    cudaDeviceProp prop; CUDA_CHECK(cudaGetDeviceProperties(&prop, dev));
     const size_t stat = 10240;  // static shared memory of decode_megakernel6 (red, redf, qh, part) + slack
     const long long room = (long long)prop.sharedMemPerBlockOptin - (long long)stat - (long long)act_b - 2 * kConsumerWarps * 8;
     int W = (int)std::min<long long>(kConsumerWarps, room / (2LL * slot));
@@ -660,6 +593,11 @@ bool LlamaDevice::build_mega6() {
     mega_smem_ = (size_t)2 * W * slot + act_b + (size_t)2 * W * 8;
     MG4_INFO("decode megakernel (generation 6): %d ops/token, %d stream warps x 2 slots x %d B, act %zu B, %zu B dynamic shared per CTA, register-resident blocks per lane %d, grid %d",
              n, W, slot, act_b, mega_smem_, mega6_nbl_, sm_count_);
+    const void *fn = mega_fn();
+    CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mega_smem_));
+    int occ = 0;
+    CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, mk6::kThreads, mega_smem_));
+    if (occ < 1) { MG4_ERR("megakernel does not fit on an SM (smem %zu)", mega_smem_); return false; }
     return true;
 }
 
@@ -692,9 +630,7 @@ void LlamaDevice::build_graph() {
     CUDA_CHECK(cudaStreamBeginCapture(stream_, cudaStreamCaptureModeThreadLocal));
     if (mega_) launch_mega();
     else {
-        if (tok_type_ == GG_Q4_K) embed_q4k_kernel<<<1, 256, 0, stream_>>>((const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, state_, x_);
-        else if (tok_type_ == GG_Q5_0 || tok_type_ == GG_Q5_1 || tok_type_ == GG_Q8_0) embed_b32_kernel<<<1, 256, 0, stream_>>>(tok_type_, (const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, state_, x_);
-        else embed_kernel<<<1, 256, 0, stream_>>>(tok_type_, (const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, state_, x_);
+        embed_rows_kernel<<<1, 256, 0, stream_>>>(tok_type_, (const unsigned char *)tok_raw_, gg_row_bytes(tok_type_, (size_t)d_.n_embd), d_.n_embd, state_->tokens, nullptr, x_);
         launch_layers(1, 1, true);
     }
     CUDA_CHECK(cudaStreamEndCapture(stream_, &g));

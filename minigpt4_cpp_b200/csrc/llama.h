@@ -47,12 +47,9 @@ public:
     ~LlamaDevice();
     bool load(const LlamaFile &f, int n_ctx, TPLink *tp);
     const LlamaDims &dims() const { return d_; }
-    // Evaluate `n` tokens / embedding rows starting at position n_past. Afterwards logits of the last row are
-    // on device and the arg-max id is known.  Returns false if the context would overflow.
-    bool eval_tokens(const int32_t *ids, int n, int n_past);
-    bool eval_embd(const float *rows_host, int n, int n_past);
-    bool eval_rows(const int32_t *ids, int n, const float *emb_host, int n_emb, int n_past);  // mixed token / embedding rows (ids < 0: row -1 - id of emb_host)
-    bool rows_mergeable() const;     // eval_rows supports this file's token-embedding type
+    // Evaluate `n` mixed token / embedding rows (ids < 0: row -1 - id of emb_host) starting at position n_past. Afterwards logits
+    // of the last row are on device and the arg-max id is known.  Returns false if the context would overflow.
+    bool eval_rows(const int32_t *ids, int n, const float *emb_host, int n_emb, int n_past);
     void logits_to_host(float *dst);   // n_vocab floats, synchronous
     int32_t argmax();                  // greedy id of the current logits (already in pinned host memory after a sync)
     void sync();
@@ -61,7 +58,7 @@ public:
     bool uses_megakernel() const { return mega_; }
     bool uses_prefill_gemm() const { return pf_ready_; }
     static constexpr int kPrefillMax = 512;   // rows per prefill pass (the reference's default n_batch)
-    int mega_generation() const { return mega_ ? mega_gen_ : 0; }
+    int mega_generation() const { return mega_ ? 6 : 0; }   // llama_mega6.cuh
     int mega_trace(long long *out, int max_values);  // debug: per-op clock64 stamps of the last megakernel launch (env MINIGPT4_B200_MEGA_TRACE)
     // one decode step through the captured CUDA graph: feeds `id` (or, if id < 0, the on-device arg-max of the
     // previous step), leaves new logits/arg-max on device.
@@ -90,11 +87,9 @@ private:
     bool pf_ready_ = false; int pf_S_e_ = 0, pf_S_ff_ = 0;
     signed char *pf_q8_ = nullptr; void *pf_sc_ = nullptr; int32_t *tok_ids_ = nullptr; void *pf_part_ = nullptr; size_t pf_part_bytes_ = 0;
     alignas(64) unsigned char pf_tmB_e_[128], pf_tmS_e_[128], pf_tmB_ff_[128], pf_tmS_ff_[128];
-    void run_chunk(int n, bool want_logits, bool from_tokens);
     void launch_layers(int nt, int ntok, bool want_logits);
     void build_graph();
     bool build_mega();               // persistent one-launch-per-token decode (homogeneous Q4_0/Q4_1, single GPU)
-    bool build_mega6();
     void launch_mega();
     const void *mega_fn() const;
     LlamaDims d_{};
@@ -120,7 +115,7 @@ private:
     unsigned long long launches_ = 0;
     int graph_kernels_ = 0;
     long long *mega_trace_ = nullptr; int mega_n_ops_ = 0;
-    int mega_gen_ = 6; void *mega6_params_ = nullptr; int mega6_nbl_ = 0;  // generation 6 (llama_mega6.cuh)
+    void *mega6_params_ = nullptr; int mega6_nbl_ = 0;  // generation 6 (llama_mega6.cuh)
     bool h_state_busy_ = false;
     bool mega_ = false; unsigned *mega_barrier_ = nullptr; size_t mega_smem_ = 0; int mega_type_ = -1;
     int sm_count_ = 148;

@@ -765,58 +765,38 @@ __device__ __forceinline__ float dequant_elem(int type, const unsigned char *row
     }
     return 0.f;
 }
-__global__ void embed_kernel(int type, const unsigned char *tok, size_t row_bytes, int E, const DeviceState *st, float *x) {
-    const int t = blockIdx.x;
-    const unsigned char *row = tok + (size_t)st->tokens[t] * row_bytes;
-    for (int i = threadIdx.x; i < E; i += blockDim.x) x[(size_t)t * E + i] = dequant_elem(type, row, i);
-}
-// the same gather for a long id list (prefill passes of up to 512 tokens; DeviceState::tokens holds 8)
-__global__ void embed_ids_kernel(int type, const unsigned char *tok, size_t row_bytes, int E, const int *ids, float *x) {
-    const int t = blockIdx.x;
-    const unsigned char *row = tok + (size_t)ids[t] * row_bytes;
-    for (int i = threadIdx.x; i < E; i += blockDim.x) x[(size_t)t * E + i] = dequant_elem(type, row, i);
-}
-// mixed rows of one prefill pass: ids[t] >= 0 = token (gather + dequantise), ids[t] < 0 = embedding row -1 - ids[t] of `emb` (the 32 image rows)
-__global__ void embed_rows_kernel(int type, const unsigned char *tok, size_t row_bytes, int E, const int *ids, const float *emb, float *x) {
-    const int t = blockIdx.x, id = ids[t];
-    if (id >= 0) {
-        const unsigned char *row = tok + (size_t)id * row_bytes;
-        for (int i = threadIdx.x; i < E; i += blockDim.x) x[(size_t)t * E + i] = dequant_elem(type, row, i);
-    } else {
-        const float *src = emb + (size_t)(-1 - id) * E;
-        for (int i = threadIdx.x; i < E; i += blockDim.x) x[(size_t)t * E + i] = src[i];
-    }
-}
-// Q4_K token-embedding rows: kept out of dequant_elem so that the kernels which inline it
-// (embed_kernel, the decode megakernel) stay byte-identical to the measured build
-__global__ void embed_q4k_kernel(const unsigned char *tok, size_t row_bytes, int E, const DeviceState *st, float *x) {
-    const int t = blockIdx.x;
-    const unsigned char *row = tok + (size_t)st->tokens[t] * row_bytes;
-    for (int i = threadIdx.x; i < E; i += blockDim.x) {
+// dequant_elem plus the token-embedding types it does not cover (Q4_K, and Q5_0 / Q5_1 / Q8_0 = ggml dequantize_row_q5_0 / q5_1 / q8_0).
+// The decode megakernel gathers through dequant_elem alone, so build_mega refuses files whose tok_embeddings need this.
+__device__ __forceinline__ float embed_elem(int type, const unsigned char *row, int i) {
+    if (type == GG_Q4_K) {
         const unsigned char *b = row + (i / 256) * 144; const int e = i % 256, sub = e / 32, l = e % 32;
         const float d = __half2float(*(const __half *)b), dmin = __half2float(*(const __half *)(b + 2));
         int sc, mn; scale_min_k4(b + 4, sub, sc, mn);
         const unsigned char qb = b[16 + (sub / 2) * 32 + l]; const int nib = (sub & 1) ? (qb >> 4) : (qb & 0xF);
-        x[(size_t)t * E + i] = (d * (float)sc) * (float)nib - dmin * (float)mn;
+        return (d * (float)sc) * (float)nib - dmin * (float)mn;
     }
+    const int j = i % 32, jj = j & 15;
+    if (type == GG_Q8_0) { const unsigned char *b = row + (i / 32) * 34; return (float)(int)(signed char)b[2 + j] * __half2float(*(const __half *)b); }
+    if (type == GG_Q5_0 || type == GG_Q5_1) {
+        const int hdr = type == GG_Q5_1 ? 4 : 2;
+        const unsigned char *b = row + (i / 32) * (hdr + 20);
+        const unsigned qh = b[hdr] | (b[hdr + 1] << 8) | (b[hdr + 2] << 16) | ((unsigned)b[hdr + 3] << 24);
+        const int q = (j < 16 ? (b[hdr + 4 + jj] & 0xF) : (b[hdr + 4 + jj] >> 4)) | (int)(((qh >> j) & 1u) << 4);
+        const float d = __half2float(*(const __half *)b);
+        return type == GG_Q5_1 ? (float)q * d + __half2float(*(const __half *)(b + 2)) : (float)(q - 16) * d;
+    }
+    return dequant_elem(type, row, i);
 }
-// token-embedding rows of Q5_0 / Q5_1 / Q8_0 files (ggml dequantize_row_q5_0 / q5_1 / q8_0), raw ggml blocks; kept out of dequant_elem (see above)
-__global__ void embed_b32_kernel(int type, const unsigned char *tok, size_t row_bytes, int E, const DeviceState *st, float *x) {
-    const int t = blockIdx.x;
-    const unsigned char *row = tok + (size_t)st->tokens[t] * row_bytes;
-    for (int i = threadIdx.x; i < E; i += blockDim.x) {
-        const int j = i % 32, jj = j & 15;
-        float v;
-        if (type == GG_Q8_0) { const unsigned char *b = row + (i / 32) * 34; v = (float)(int)(signed char)b[2 + j] * __half2float(*(const __half *)b); }
-        else {
-            const int hdr = type == GG_Q5_1 ? 4 : 2;
-            const unsigned char *b = row + (i / 32) * (hdr + 20);
-            const unsigned qh = b[hdr] | (b[hdr + 1] << 8) | (b[hdr + 2] << 16) | ((unsigned)b[hdr + 3] << 24);
-            const int q = (j < 16 ? (b[hdr + 4 + jj] & 0xF) : (b[hdr + 4 + jj] >> 4)) | (int)(((qh >> j) & 1u) << 4);
-            const float d = __half2float(*(const __half *)b);
-            v = type == GG_Q5_1 ? (float)q * d + __half2float(*(const __half *)(b + 2)) : (float)(q - 16) * d;
-        }
-        x[(size_t)t * E + i] = v;
+// rows of one pass: ids[t] >= 0 = token (gather + dequantise), ids[t] < 0 = embedding row -1 - ids[t] of `emb` (the 32 image rows).
+// The per-op decode graph passes DeviceState::tokens as `ids` (one row, no `emb`).
+__global__ void embed_rows_kernel(int type, const unsigned char *tok, size_t row_bytes, int E, const int *ids, const float *emb, float *x) {
+    const int t = blockIdx.x, id = ids[t];
+    if (id >= 0) {
+        const unsigned char *row = tok + (size_t)id * row_bytes;
+        for (int i = threadIdx.x; i < E; i += blockDim.x) x[(size_t)t * E + i] = embed_elem(type, row, i);
+    } else {
+        const float *src = emb + (size_t)(-1 - id) * E;
+        for (int i = threadIdx.x; i < E; i += blockDim.x) x[(size_t)t * E + i] = src[i];
     }
 }
 __global__ void finalize_kernel(DeviceState *st, int want_logits, int *argmax_out) {

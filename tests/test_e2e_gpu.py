@@ -146,27 +146,32 @@ def test_batched_encode_equals_single_encodes(lib, ext, mg, tiny, big_llm):
     lib.minigpt4_free(c)
 
 
+def check_queued_pieces(ext, llm):
+    """The pieces of one chat turn queued (one pass over the weights at the end) versus flushed one by one: same logits, same greedy ids."""
+    c1, c2 = ext.llm_load(llm, n_ctx=512), ext.llm_load(llm, n_ctx=512)
+    rng = np.random.default_rng(3)
+    rows = rng.standard_normal((32, ext.L.minigpt4_b200_n_embd(c1.ptr))).astype(np.float32)
+    pieces = [("t", list(range(5, 25))), ("t", [7, 9, 11]), ("e", rows), ("t", [4]), ("t", list(range(30, 47))), ("t", [3, 3, 8])]
+    for kind, p in pieces:
+        (ext.eval_tokens if kind == "t" else ext.eval_embd)(c1, p)                      # queued: one pass over the weights at the end
+        (ext.eval_tokens if kind == "t" else ext.eval_embd)(c2, p); ext.flush(c2)      # forced: one pass per piece
+    assert ext.n_past(c1) == ext.n_past(c2) == sum(len(p) for _, p in pieces)
+    assert np.array_equal(ext.logits(c1), ext.logits(c2))
+    a, b = [], []
+    for _ in range(6):
+        t1, t2 = ext.greedy_id(c1), ext.greedy_id(c2); a.append(t1); b.append(t2)
+        ext.eval_tokens(c1, [t1]); ext.eval_tokens(c2, [t2])
+    assert a == b
+    with pytest.raises(RuntimeError, match="FailedToAddString"):   # validated when queued, not when flushed
+        ext.eval_tokens(c1, [10 ** 9])
+    ext.base.minigpt4_free(c1); ext.base.minigpt4_free(c2)
+
+
 def test_queued_prompt_pieces_equal_piecewise_evaluation(ext, tiny):
     """The engine queues consecutive add_tokens / add_embedding calls and evaluates them in one pass (the reference evaluates each piece on its own,
     minigpt4.cpp:2365-2415).  Rows are batch invariant, so the logits must not change by a single bit; errors are still raised at queue time."""
     for wt in ("q4_1", "q5_k"):
-        c1, c2 = ext.llm_load(tiny[wt], n_ctx=512), ext.llm_load(tiny[wt], n_ctx=512)
-        rng = np.random.default_rng(3)
-        rows = rng.standard_normal((32, ext.L.minigpt4_b200_n_embd(c1.ptr))).astype(np.float32)
-        pieces = [("t", list(range(5, 25))), ("t", [7, 9, 11]), ("e", rows), ("t", [4]), ("t", list(range(30, 47))), ("t", [3, 3, 8])]
-        for kind, p in pieces:
-            (ext.eval_tokens if kind == "t" else ext.eval_embd)(c1, p)                      # queued: one pass over the weights at the end
-            (ext.eval_tokens if kind == "t" else ext.eval_embd)(c2, p); ext.flush(c2)      # forced: one pass per piece
-        assert ext.n_past(c1) == ext.n_past(c2) == sum(len(p) for _, p in pieces)
-        assert np.array_equal(ext.logits(c1), ext.logits(c2))
-        a, b = [], []
-        for _ in range(6):
-            t1, t2 = ext.greedy_id(c1), ext.greedy_id(c2); a.append(t1); b.append(t2)
-            ext.eval_tokens(c1, [t1]); ext.eval_tokens(c2, [t2])
-        assert a == b
-        with pytest.raises(RuntimeError, match="FailedToAddString"):   # validated when queued, not when flushed
-            ext.eval_tokens(c1, [10 ** 9])
-        ext.base.minigpt4_free(c1); ext.base.minigpt4_free(c2)
+        check_queued_pieces(ext, tiny[wt])
 
 
 def test_context_overflow_is_an_error(ext, tiny):
